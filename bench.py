@@ -30,6 +30,12 @@ Other workloads (secondary lines, same JSON contract; the driver runs the defaul
   --workload c5   BASELINE configs[4]: 50 views 4032x3024, pass 1 + ONE geometric-consistency pass: per step every rank
                   estimates its views, all-gathers the depth-maps (ncclAllGather, timed separately with CUDA events),
                   re-estimates them with the neighbours' depth-maps, and rank 0 gathers the result.
+
+--dump-outputs DIR
+  after the timed steps, rank 0 writes the maps the timed path returned for its reference views in the last step, at one fixed,
+  seeded sample of pixels (the same for every view, 32 MB of data at most): DIR/depth.npy [V, P], normal.npy [V, P, 3],
+  conf.npy [V, P] and views.npy [V, P, 4], float32.  The scene is seeded, so two builds given the same arguments can be compared
+  output for output.
 """
 from __future__ import annotations
 
@@ -43,6 +49,8 @@ import time
 
 import numpy as np
 
+# the tree the benchmark runs from may be read-only: nothing is written into it
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
 	sys.path.insert(0, ROOT)
@@ -63,7 +71,30 @@ def parse():
 	ap.add_argument("--no-cpu-baseline", action="store_true")
 	ap.add_argument("--no-sgm", action="store_true")
 	ap.add_argument("--small", action="store_true", help="developer mode: 640x360 scene")
-	return ap.parse_args()
+	ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed sample of the last timed step's maps to DIR/*.npy")
+	args = ap.parse_args()
+	if args.steps < 1:
+		ap.error("--steps must be at least 1")
+	if args.dump_outputs and args.impl == "reference":
+		ap.error("--dump-outputs writes the engine's maps: not with --impl reference")
+	return args
+
+
+DUMP_BYTES = 32_000_000
+
+
+def dump_outputs(directory, stack, views):
+	"""DIR/<map>.npy of the maps `stack` holds for `views`, at a fixed, seeded sample of pixels (sorted, the same for every
+	view) sized to keep the four files within DUMP_BYTES."""
+	import torch
+	hw = stack.h*stack.w
+	n = min(hw, DUMP_BYTES//(len(views)*9*4))   # 9 floats per pixel: depth, normal, conf, 4 view ids
+	idx = torch.from_numpy(np.sort(np.random.RandomState(0).choice(hw, n, replace=False))).to(stack.depth.device)
+	slots = torch.tensor([stack.slot(v) for v in views], device=stack.depth.device)
+	os.makedirs(directory, exist_ok=True)
+	for name, t, c in (("depth", stack.depth, 1), ("normal", stack.normal, 3), ("conf", stack.conf, 1), ("views", stack.views, 4)):
+		a = t.view(t.shape[0], hw, c)[:, idx][slots].float().cpu().numpy()
+		np.save(os.path.join(directory, name+".npy"), a[..., 0] if c == 1 else a)
 
 
 class ClockSampler:
@@ -426,6 +457,8 @@ def main():
 	ms_res, _ = timed(step_resident, args.steps, args.warmup)
 	n_launch = launches[0]*args.steps//(args.steps+args.warmup)
 	clocks = sampler.stop() if rank == 0 else None
+	if args.dump_outputs and rank == 0:
+		dump_outputs(args.dump_outputs, stack, mine)
 	ms_e2e, (h2d, d2h) = timed(step_e2e, args.steps, max(1, args.warmup//3))
 	mpix_step = N_VIEWS*w*h/1e6*world
 	value = mpix_step/(ms_res/args.steps/1e3)
@@ -580,6 +613,8 @@ def run_scene_workload(args, dev, rank, world, local_rank, peak):
 	ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
 	if world > 1: dist.all_reduce(ms, op=dist.ReduceOp.MAX)
 	clocks = sampler.stop() if rank == 0 else None
+	if args.dump_outputs and rank == 0:
+		dump_outputs(args.dump_outputs, stack, stack.mine)
 	ms_step = float(ms.item())/args.steps
 	passes = 2 if c5 else 1
 	value = n_views*w*h/1e6/(ms_step/1e3)

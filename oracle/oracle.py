@@ -5,9 +5,12 @@ import this module.  The product package openmvs_b200 never does.
 """
 from __future__ import annotations
 
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -38,28 +41,20 @@ def build(force: bool = False) -> str:
 	return so
 
 
-def _cpu_model() -> str:
-	try:
-		for line in open("/proc/cpuinfo"):
-			if line.startswith("model name"):
-				return line.split(":", 1)[1].strip()
-	except Exception:
-		pass
-	return "unknown"
+_FAST_SO = None
 
 
 def build_fast() -> str:
 	"""Throughput build of the same sources (-O3 -march=native, FP contraction allowed) for the CPU baseline of bench.py.  It is
-	compiled on the machine that runs it (the marker file names the CPU it was built for): -march=native code must not travel."""
-	so = os.path.join(_HERE, "liboracle_fast.so")
-	tag = os.path.join(_HERE, "liboracle_fast.cpu")
-	srcs = [os.path.join(_HERE, f) for f in ("pm_oracle.cpp", "sgm_oracle.cpp", "filter_oracle.cpp", "oracle.h")]
-	fresh = os.path.exists(so) and os.path.exists(tag) and open(tag).read() == _cpu_model() and all(
-		os.path.getmtime(s) <= os.path.getmtime(so) for s in srcs)
-	if not fresh:
-		subprocess.check_call(["make", "-C", _HERE, "-s", "-B", "liboracle_fast.so"])
-		open(tag, "w").write(_cpu_model())
-	return so
+	compiled once per process into a temporary directory: -march=native code must not travel, and the tree may be read-only."""
+	global _FAST_SO
+	if _FAST_SO is None:
+		tmp = tempfile.mkdtemp(prefix="oracle_fast_")
+		atexit.register(shutil.rmtree, tmp, True)
+		so = os.path.join(tmp, "liboracle_fast.so")
+		subprocess.check_call(["make", "-C", _HERE, "-s", "FAST_SO="+so, so])
+		_FAST_SO = so
+	return _FAST_SO
 
 
 _LIBS = {}

@@ -1,12 +1,12 @@
-"""Every `path:line` citation of the reference in the sources, headers and docs points at an existing file and
-line range of /root/reference (skipped where the reference is not mounted, e.g. on the GPU box)."""
+"""Every `path:line` citation of the reference in the sources, headers and docs points at an existing file and line range of
+the reference.  The reference's files and their line counts are stored in tests/golden/reference_line_counts.json
+(tests/golden/make_reference_goldens.py)."""
+import json
 import os
 import re
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+LINE_COUNTS = os.path.join(ROOT, "tests", "golden", "reference_line_counts.json")
 # full paths (libs/MVS/DepthMap.cpp:465-564) and bare file names (DepthMap.cpp:465-564; resolved through the reference tree)
 PAT = re.compile(r"(?<![A-Za-z0-9_/.-])((?:(?:libs|apps|scripts|docs|build)/)?[A-Za-z0-9_./+-]*[A-Za-z0-9_+-]+\.(?:cpp|h|inl|cu|txt|yml))`?:(\d+)(?:-(\d+))?")
 OWN = ("pm_kernels.cu", "capi.cu", "sgm_kernels.cu", "filter_kernels.cu", "resize_kernels.cu", "b200mvs.h", "oracle.h", "pm_oracle.cpp",
@@ -22,13 +22,10 @@ def _files():
 
 
 def test_reference_citations_resolve():
-	if not os.path.isdir(REF):
-		pytest.skip("reference not mounted")
+	lengths = json.load(open(LINE_COUNTS))
 	index = {}
-	for dp, _, fn in os.walk(REF):
-		for f in fn:
-			index.setdefault(f, []).append(os.path.relpath(os.path.join(dp, f), REF))
-	lengths = {}
+	for rel in lengths:
+		index.setdefault(os.path.basename(rel), []).append(rel)
 	bad = []
 	n = 0
 	for path in _files():
@@ -42,11 +39,8 @@ def test_reference_citations_resolve():
 					if not cands: bad.append("%s cites %s: no such file in the reference" % (os.path.relpath(path, ROOT), rel))
 					continue  # ambiguous bare names (CMakeLists.txt) are not checked
 				rel = cands[0]
-			full = os.path.join(REF, rel)
-			if rel not in lengths:
-				lengths[rel] = sum(1 for _ in open(full, errors="replace")) if os.path.isfile(full) else -1
 			n += 1
-			if lengths[rel] < 0 or not (1 <= a <= b <= lengths[rel]):
-				bad.append("%s cites %s:%d-%d (%s)" % (os.path.relpath(path, ROOT), rel, a, b, "missing file" if lengths[rel] < 0 else "%d lines" % lengths[rel]))
+			if rel not in lengths or not (1 <= a <= b <= lengths[rel]):
+				bad.append("%s cites %s:%d-%d (%s)" % (os.path.relpath(path, ROOT), rel, a, b, "%d lines" % lengths[rel] if rel in lengths else "missing file"))
 	assert n > 200
 	assert not bad, "\n".join(bad[:20])

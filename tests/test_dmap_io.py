@@ -1,9 +1,7 @@
 """.dmap writer/reader: byte layout of HeaderDepthDataRaw (libs/MVS/Interface.h:773-792), round trip,
-and — when the reference tree is present (this container only) — our files read back by the
-reference's own Python reader scripts/python/MvsUtils.py:loadDMAP."""
+and our files as the reference's own Python reader scripts/python/MvsUtils.py:loadDMAP read them (stored fixture)."""
 import os
 import struct
-import sys
 
 import numpy as np
 import pytest
@@ -48,20 +46,22 @@ def test_byte_layout_and_round_trip(tmp_path):
 		dmap_io.ExportDepthDataRaw(p, "x.jpg", [0], (17, 12), K, R, C, 1, 2, depth)
 
 
-def test_reference_reader_reads_our_files(tmp_path):
-	ref = "/root/reference/scripts/python"
-	if not os.path.exists(os.path.join(ref, "MvsUtils.py")):
-		pytest.skip("reference tree not present (GPU box)")
-	sys.path.insert(0, ref)
-	try:
-		from MvsUtils import loadDMAP
-	finally:
-		sys.path.remove(ref)
+def write_reader_case(directory):
+	"""The file whose reading by the reference's reader is stored in tests/golden/dmap_reference_reader.npz."""
 	rng = np.random.RandomState(1)
 	depth, normal, conf, views, K, R, C = _sample(rng)
-	p = str(tmp_path/"depth0001.dmap")
-	dmap_io.ExportDepthDataRaw(p, str(tmp_path/"img.jpg"), [7, 2, 5, 9], (17, 12), K, R, C, 0.25, 7.5, depth, normal, conf, views)
-	d = loadDMAP(p)
+	p = os.path.join(str(directory), "depth0001.dmap")
+	dmap_io.ExportDepthDataRaw(p, os.path.join(str(directory), "img.jpg"), [7, 2, 5, 9], (17, 12), K, R, C, 0.25, 7.5, depth, normal, conf, views)
+	return p, (depth, normal, conf, views, K, R, C)
+
+
+def test_reference_reader_reads_our_files(tmp_path):
+	"""What the writer produces, read by the reference's own reader MvsUtils.py:loadDMAP (scripts/python of the reference).  The
+	reader's result on this file is stored in tests/golden/dmap_reference_reader.npz (tests/golden/make_reference_goldens.py):
+	the writer must still produce that file byte for byte, and what the reader read from it must be what was written."""
+	p, (depth, normal, conf, views, K, R, C) = write_reader_case(tmp_path)
+	d = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "dmap_reference_reader.npz"))
+	assert open(p, "rb").read() == d["dmap"].tobytes()
 	assert d["depth_width"] == 17 and d["depth_height"] == 12 and d["reference_view_id"] == 7 and list(d["neighbor_view_ids"]) == [2, 5, 9]
 	assert np.array_equal(d["depth_map"], depth) and np.array_equal(d["normal_map"], normal)
 	assert np.array_equal(d["confidence_map"], conf) and np.array_equal(d["views_map"], views)
