@@ -10,8 +10,9 @@
 // same-colour pixels of one image row (64-pixel span), so the homography-warped taps of
 // the 32 lanes fall on 2-3 cache lines of two neighbour-image rows.  The bilateral
 // weights of the 5x5 reference patch are computed once per pixel and sweep from a reference
-// tile that TMA stages into shared memory, kept in shared memory as float2{w, tw}[tap][thread]
-// (80 registers per thread, 24 warps per SM) and reused by every hypothesis x view.
+// tile that TMA stages into shared memory, kept in tensor memory (TMEM, one lane per pixel,
+// read by tcgen05.ld off the L1 data pipe that the texel gathers bind) and reused by every
+// hypothesis x view (80 registers per thread, 24 warps per SM).
 // All four 4-neighbours belong to the other colour, so in-place updates are race-free.
 // Measured design history and the variants that were dropped: DESIGN.md section 5.1.
 #include "pm_common.cuh"
@@ -26,13 +27,51 @@ constexpr int BLOCK_Y = 8;
 
 constexpr int NTHREADS = BLOCK_X*BLOCK_Y;
 
-// bilateral weights of the 5x5 reference patch (WeightedPatchFix<25>, DepthMap.h:145-155), kept in shared
-// memory as float2{w,tw}[tap][thread] (conflict-free LDS.64): 50 registers per thread less than a register copy
+// Bilateral weights of the 5x5 reference patch (WeightedPatchFix<25>, DepthMap.h:145-155): 50 registers per thread
+// less than a register copy.  Two homes with one interface: the scoring code reads tap row i as r[2j] = w, r[2j+1] = tw
+// (j = 0..4) through load_row(i, r) and may use r only after wait_row(r).
+// PatchW (pass A): shared memory, float2{w,tw}[tap][thread] (conflict-free LDS.64).
 struct PatchW {
 	float2* s; // &smem[threadIndex]; tap k at s[k*NTHREADS]
 	float sumW, normSq0;
 	__device__ __forceinline__ void set(int k, float a, float b) { s[k*NTHREADS] = make_float2(a, b); }
-	__device__ __forceinline__ float2 get(int k) const { return s[k*NTHREADS]; }
+	__device__ __forceinline__ void load_row(int i, uint32_t (&r)[10]) const {
+		#pragma unroll
+		for (int j = 0; j < 5; ++j) {
+			const float2 v = s[(5*i+j)*NTHREADS];
+			r[2*j] = __float_as_uint(v.x); r[2*j+1] = __float_as_uint(v.y);
+		}
+	}
+	__device__ __forceinline__ void wait_row(uint32_t (&)[10]) const {}
+};
+
+// PatchT (the sweep): tensor memory, one TMEM lane per pixel.  A warp reaches only the 32 lanes of its quarter (warp % 4),
+// so warps w and w+4 share a quarter at column blocks 0 and 64 of the CTA's 128 columns.  Columns of a block: taps 0..3 of
+// row i at 8i..8i+7 ({w, tw} per tap), tap 4 of row i at 40+2i..41+2i.  A tap row is read as one tcgen05.ld .x4 per tap pair
+// and one .x2 for the fifth tap, each at its natural alignment (measured 1 % faster per launch than one .x8 + one .x2 per row,
+// DESIGN.md §5.1).  tcgen05.ld/st are .sync.aligned: every lane of the warp executes them.
+constexpr uint32_t SWEEP_TMEM_COLS = 128;
+struct PatchT {
+	uint32_t t; // TMEM address: lane quarter << 16 | column block
+	float sumW, normSq0;
+	__device__ __forceinline__ static uint32_t col(int k) { const int i = k/5, j = k%5; return j < 4 ? 8*i+2*j : 40+2*i; }
+	__device__ __forceinline__ void set(int k, float a, float b) {
+		asm volatile("tcgen05.st.sync.aligned.32x32b.x2.b32 [%0], {%1, %2};"
+			:: "r"(t+col(k)), "r"(__float_as_uint(a)), "r"(__float_as_uint(b)) : "memory");
+	}
+	// volatile: the loads must stay behind the fill's tcgen05.wait::st and must not be hoisted out of the view loop
+	__device__ __forceinline__ void load_row(int i, uint32_t (&r)[10]) const {
+		asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];"
+			: "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(t+8*i));
+		asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];"
+			: "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]) : "r"(t+8*i+4));
+		asm volatile("tcgen05.ld.sync.aligned.32x32b.x2.b32 {%0, %1}, [%2];" : "=r"(r[8]), "=r"(r[9]) : "r"(t+40+2*i));
+	}
+	// the registers of an issued tcgen05.ld are undefined until tcgen05.wait::ld: tie them to the wait
+	__device__ __forceinline__ void wait_row(uint32_t (&r)[10]) const {
+		asm volatile("tcgen05.wait::ld.sync.aligned;"
+			: "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]), "+r"(r[8]), "+r"(r[9]));
+	}
 };
 
 // ---- TMA staging of the reference tile ---------------------------------------------------------
@@ -68,7 +107,8 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, i
 }
 
 // FillPixelPatch + GetWeight from the staged tile; (lx, ly) = pixel position inside the tile
-__device__ __forceinline__ void fill_patch_tile(const float* __restrict__ tile, int lx, int ly, PatchW& p) {
+template <class PW>
+__device__ __forceinline__ void fill_patch_tile(const float* __restrict__ tile, int lx, int ly, PW& p) {
 	const float sigmaColor = -1.f/(2.f*0.1f*0.1f);
 	const float sigmaSpatial = -1.f/(2.f*9.f);
 	const float center = tile[ly*TILE_W + lx];
@@ -103,7 +143,8 @@ __device__ __forceinline__ void fill_patch_tile(const float* __restrict__ tile, 
 
 // FillPixelPatch + GetWeight (DepthMap.cpp:422-462, DepthMap.h:403-412) from global memory (pass A, and
 // the sweep when no TMA descriptor is available)
-__device__ __forceinline__ void fill_patch(const float* __restrict__ img, int pitch, int x, int y, PatchW& p) {
+template <class PW>
+__device__ __forceinline__ void fill_patch(const float* __restrict__ img, int pitch, int x, int y, PW& p) {
 	const float sigmaColor = -1.f/(2.f*0.1f*0.1f);
 	const float sigmaSpatial = -1.f/(2.f*9.f);
 	const float center = __ldg(img + (size_t)y*pitch + x);
@@ -198,9 +239,10 @@ __device__ __forceinline__ void fetch_texels(const void* __restrict__ tex, int p
 // PACK: taps evaluated two at a time with the packed fp32 instructions of sm_100 (FMUL2 / FFMA2 through
 // __fmul2_rn / __ffma2_rn): identical roundings (whole-run output bit-identical to the scalar form, photometric
 // and geometric passes), about 10 % fewer issue slots per 25 taps.  PACK = false is the debug form.
-template <bool PACK, bool GEOM>
-__device__ __forceinline__ float score_view(const PMParams& P, const PMView& V, const PatchW& pt,
-	float fx, float fy, float X0x, float X0y, const Hyp& h, float priorF, float priorD)
+// have = false: a lane that only keeps its warp converged (TMEM loads are warp-collective); it runs as a rejected lane.
+template <bool PACK, bool GEOM, class PW>
+__device__ __forceinline__ float score_view(const PMParams& P, const PMView& V, const PW& pt,
+	float fx, float fy, float X0x, float X0y, const Hyp& h, float priorF, float priorD, bool have)
 {
 	// H = A + Hm (n^T Kref^-1)/(n.X0 d); columns 0/1 and the centre point H*(x,y,1)
 	float c0x = fmaf(V.Hm[0], h.ms.x, V.A[0]), c0y = fmaf(V.Hm[1], h.ms.x, V.A[3]), c0z = fmaf(V.Hm[2], h.ms.x, V.A[6]);
@@ -222,7 +264,7 @@ __device__ __forceinline__ float score_view(const PMParams& P, const PMView& V, 
 		const float i0 = fast_rcp(bz), i1 = fast_rcp(z1), i2 = fast_rcp(z2), i3 = fast_rcp(z3);
 		const float pxmin = fminf(fminf(bx*i0, x1*i1), fminf(x2*i2, x3*i3)), pxmax = fmaxf(fmaxf(bx*i0, x1*i1), fmaxf(x2*i2, x3*i3));
 		const float pymin = fminf(fminf(by*i0, y1*i1), fminf(y2*i2, y3*i3)), pymax = fmaxf(fmaxf(by*i0, y1*i1), fmaxf(y2*i2, y3*i3));
-		ok = (zmin > 0.f || zmax < 0.f) && pxmin >= 1.f && pymin >= 1.f && pxmax <= xmax && pymax <= ymax;
+		ok = have && (zmin > 0.f || zmax < 0.f) && pxmin >= 1.f && pymin >= 1.f && pxmax <= xmax && pymax <= ymax;
 		// NaN anywhere makes a comparison false (fminf/fmaxf drop NaNs, so test them explicitly)
 		ok = ok && (bx*i0 == bx*i0) && (x1*i1 == x1*i1) && (x2*i2 == x2*i2) && (x3*i3 == x3*i3)
 		        && (by*i0 == by*i0) && (y1*i1 == y1*i1) && (y2*i2 == y2*i2) && (y3*i3 == y3*i3);
@@ -239,6 +281,8 @@ __device__ __forceinline__ float score_view(const PMParams& P, const PMView& V, 
 	#pragma unroll
 	for (int i = 0; i < 5; ++i) {
 		float X = bx, Y = by, Z = bz;
+		uint32_t wr[10]; // weights of tap row i, in flight while the row's texels are fetched
+		pt.load_row(i, wr);
 		#pragma unroll
 		for (int j = 0; j < 5; j += 2) {
 			const bool two = j+1 < 5;
@@ -270,13 +314,15 @@ __device__ __forceinline__ float score_view(const PMParams& P, const PMView& V, 
 				BOT = make_float2(fmaf(AX.x, V11.x-V01.x, V01.x), fmaf(AX.y, V11.y-V01.y, V01.y));
 				VV = make_float2(fmaf(AY.x, BOT.x-TOP.x, TOP.x), fmaf(AY.y, BOT.y-TOP.y, TOP.y));
 			}
+			if (j == 0)
+				pt.wait_row(wr);
 			{
-				const float2 wk = pt.get(i*5+j);
+				const float2 wk = make_float2(__uint_as_float(wr[2*j]), __uint_as_float(wr[2*j+1]));
 				const float vw = VV.x*wk.x;
 				sum += vw; sumSq = fmaf(VV.x, vw, sumSq); num = fmaf(VV.x, wk.y, num);
 			}
 			if (two) {
-				const float2 wk = pt.get(i*5+j+1);
+				const float2 wk = make_float2(__uint_as_float(wr[2*j+2]), __uint_as_float(wr[2*j+3]));
 				const float vw = VV.y*wk.x;
 				sum += vw; sumSq = fmaf(VV.y, vw, sumSq); num = fmaf(VV.y, wk.y, num);
 			}
@@ -327,15 +373,15 @@ __device__ __forceinline__ float score_view(const PMParams& P, const PMView& V, 
 }
 
 // ScorePixel (DepthMap.cpp:567-626): MINMEAN over the views; also reports the two best views
-template <bool PACK, bool GEOM>
-__device__ __forceinline__ float score_pixel(const PMParams& P, const PatchW& pt,
-	float fx, float fy, float X0x, float X0y, const Hyp& h, float priorF, float priorD, uint32_t& best)
+template <bool PACK, bool GEOM, class PW>
+__device__ __forceinline__ float score_pixel(const PMParams& P, const PW& pt,
+	float fx, float fy, float X0x, float X0y, const Hyp& h, float priorF, float priorD, bool have, uint32_t& best)
 {
 	float s0 = CUDART_INF_F, s1 = CUDART_INF_F;
 	int i0 = 255, i1 = 255;
 	#pragma unroll 1
 	for (int v = 0; v < P.nViews; ++v) {
-		const float s = score_view<PACK, GEOM>(P, P.views[v], pt, fx, fy, X0x, X0y, h, priorF, priorD);
+		const float s = score_view<PACK, GEOM>(P, P.views[v], pt, fx, fy, X0x, X0y, h, priorF, priorD, have);
 		if (s < s0) { s1 = s0; i1 = i0; s0 = s; i0 = v; }
 		else if (s < s1) { s1 = s; i1 = v; }
 	}
@@ -469,7 +515,7 @@ pm_score_kernel(const __grid_constant__ PMParams P)
 	Hyp h;
 	make_hyp(P, X0x, X0y, d, n, cl, false, h);
 	uint32_t best;
-	const float c = score_pixel<PACK, GEOM>(P, pt, fx, fy, X0x, X0y, h, priorF, priorD, best);
+	const float c = score_pixel<PACK, GEOM>(P, pt, fx, fy, X0x, X0y, h, priorF, priorD, true, best);
 	P.plane[idx] = make_float4(n.x, n.y, n.z, d);
 	P.cost[idx] = c;
 	if (P.bestViews) P.bestViews[idx] = best;
@@ -485,49 +531,28 @@ pm_score_kernel(const __grid_constant__ PMParams P)
 //      all kept their plane in their last update (they lost against this pixel one sweep ago) — P.skipUnchanged;
 //   3. the refinement state machine (DepthMap.cpp:800-852).
 // Every lane keeps its own to-do list of directions, so a warp runs max-over-lanes(list length) test steps.
-// MINB: resident CTAs per SM the register allocation aims at: 3 (80 registers, the default) or 4 (64 registers: one more CTA of
-// latency hiding against more spill traffic — b200mvs_debug.sweepFourCtas, measured in profiles/pm_4ctas_r02.txt: slower)
-template <bool PACK, bool GEOM, int MINB>
-__global__ void __launch_bounds__(BLOCK_X*BLOCK_Y, MINB)
-pm_sweep_kernel(const __grid_constant__ PMParams P, const __grid_constant__ CUtensorMap tmapRef)
+//
+// The TMEM loads of the scoring code are warp-collective, so every lane of a warp that has a pixel to update runs the whole
+// loop: a lane whose pixel is on the border, masked out or textureless is not `live` (it never has a hypothesis and stores
+// nothing), and a lane without a hypothesis in a step scores its current plane as a rejected lane and drops the result.
+template <bool PACK, bool GEOM>
+__device__ __forceinline__ void sweep_pixel(const PMParams& P, const float* __restrict__ tile, uint32_t tmem, int x, int y, bool live)
 {
-	extern __shared__ __align__(128) unsigned char smemRaw[];
-	// [ patch weights | reference tile | mbarrier ]
-	float2* smemW = (float2*)smemRaw;
-	float* tile = (float*)(smemRaw + PM_TEXELS*NTHREADS*sizeof(float2));
-	uint64_t* bar = (uint64_t*)(tile + TILE_W*TILE_H);
-	const int tid = threadIdx.y*BLOCK_X + threadIdx.x;
-	if (P.tma) {
-		if (tid == 0) {
-			mbar_init(bar, 1);
-			asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); // make the init visible to the async proxy
-		}
-		__syncthreads();
-		if (tid == 0) {
-			mbar_expect_tx(bar, TILE_BYTES);
-			tma_load_2d(tile, &tmapRef, (int)blockIdx.x*(2*BLOCK_X)-PM_HALF, (int)blockIdx.y*BLOCK_Y-PM_HALF, bar);
-		}
-		mbar_wait(bar, 0);
-	}
-	const int y = blockIdx.y*BLOCK_Y + threadIdx.y;
-	const int x = blockIdx.x*(2*BLOCK_X) + 2*threadIdx.x + ((y+P.colour)&1);
-	if (x < PM_HALF || y < PM_HALF || x >= P.W-PM_HALF || y >= P.H-PM_HALF)
-		return;
-	if (P.mask && P.mask[(size_t)y*P.maskPitch + x] == 0)
-		return;
 	const int W = P.W, H = P.H;
 	const size_t idx = (size_t)y*W + x;
-	PatchW pt;
-	pt.s = smemW + tid;
+	PatchT pt;
+	pt.t = tmem;
+	// a dead lane fills from any in-image patch (the warp has a live pixel, so the image is at least 9 x 9)
 	if (P.tma)
 		fill_patch_tile(tile, 2*(int)threadIdx.x + ((y+P.colour)&1) + PM_HALF, (int)threadIdx.y + PM_HALF, pt);
 	else
-		fill_patch(P.img0, P.pitch0, x, y, pt);
+		fill_patch(P.img0, P.pitch0, live ? x : PM_HALF, live ? y : PM_HALF, pt);
+	asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
 	float priorD = 0.f, priorF = 0.f;
-	if (P.lowres)
+	if (live && P.lowres)
 		priorD = fmaxf(__ldg(P.lowres + idx), 0.f);
 	if (pt.normSq0 < P.thMagnitudeSq && !(priorD > 0.f))
-		return;
+		live = false;
 	if (priorD > 0.f)
 		priorF = expf(pt.normSq0*(-1.f/0.02f));
 	const float fx = float(x), fy = float(y);
@@ -545,7 +570,7 @@ pm_sweep_kernel(const __grid_constant__ PMParams P, const __grid_constant__ CUte
 		const int kk = dir ? (k^2) : k;
 		const int ox = (kk == 0) ? -1 : (kk == 2) ? 1 : 0;
 		const int oy = (kk == 1) ? -1 : (kk == 3) ? 1 : 0;
-		const bool ok = (kk == 0) ? (x > PM_HALF) : (kk == 1) ? (y > PM_HALF) : (kk == 2) ? (x < W-PM_HALF) : (y < H-PM_HALF);
+		const bool ok = live && ((kk == 0) ? (x > PM_HALF) : (kk == 1) ? (y > PM_HALF) : (kk == 2) ? (x < W-PM_HALF) : (y < H-PM_HALF));
 		cl.d[k] = 0.f; cl.n[k] = make_float3(0.f, 0.f, 0.f); cl.rx[k] = 0.f; cl.ry[k] = 0.f;
 		if (ok) {
 			const size_t nidx = (size_t)(y+oy)*W + (x+ox);
@@ -577,11 +602,11 @@ pm_sweep_kernel(const __grid_constant__ PMParams P, const __grid_constant__ CUte
 			}
 		}
 	}
-	const float4 pl = P.plane[idx];
-	float conf = fabsf(P.cost[idx]);
+	const float4 pl = live ? P.plane[idx] : make_float4(0.f, 0.f, -1.f, 1.f); // a dead lane: a finite plane to score
+	float conf = live ? fabsf(P.cost[idx]) : 0.f;
 	float depth = pl.w;
 	float3 normal = make_float3(pl.x, pl.y, pl.z);
-	uint32_t bestViews = P.bestViews ? P.bestViews[idx] : 0xFFFFFFFFu;
+	uint32_t bestViews = (live && P.bestViews) ? P.bestViews[idx] : 0xFFFFFFFFu;
 
 	// ---- propagation (DepthMap.cpp:775-799), then the refinement state machine (DepthMap.cpp:800-852) ----
 	// One loop and one copy of the scoring code for both: a lane first pops its propagation candidates, then runs its
@@ -594,8 +619,8 @@ pm_sweep_kernel(const __grid_constant__ PMParams P, const __grid_constant__ CUte
 	const int nRl = P.evalCap > 0 ? min(nR, max(P.evalCap-__popc(todo), 1)) : nR;
 	const uint2 key = make_uint2(P.seed, 0xB200C0DEu);
 	const uint32_t phase = 1u + (uint32_t)P.sweep;
-	int mode = 0;               // 0 undecided, 1 restart (fully random), 2 refine, 3 done
-	bool entered = false;       // the state machine has taken its first decision
+	int mode = live ? 0 : 3;    // 0 undecided, 1 restart (fully random), 2 refine, 3 done
+	bool entered = !live;       // the state machine has taken its first decision
 	bool useClose = true;
 	unsigned idxScale = 0;
 	float scaleRange = 1.f, depthRange = 0.f, pa = 0.f, pb = 0.f;
@@ -673,25 +698,70 @@ pm_sweep_kernel(const __grid_constant__ PMParams P, const __grid_constant__ CUte
 			break;
 		if (!__any_sync(__activemask(), have))
 			continue;
-		if (have) {
-			Hyp h;
-			make_hyp(P, X0x, X0y, hd, hn, cl, uc, h);
-			uint32_t bv;
-			const float nconf = score_pixel<PACK, GEOM>(P, pt, fx, fy, X0x, X0y, h, priorF, priorD, bv);
-			if (conf > nconf) {
-				conf = nconf; depth = hd; normal = hn; bestViews = bv;
-				if (isRefine) {
-					pa = na; pb = nb;
-					++idxScale;
-					scaleRange = pow2neg(idxScale);
-				}
+		if (!have) { hd = depth; hn = normal; }
+		Hyp h;
+		make_hyp(P, X0x, X0y, hd, hn, cl, uc, h);
+		uint32_t bv;
+		const float nconf = score_pixel<PACK, GEOM>(P, pt, fx, fy, X0x, X0y, h, priorF, priorD, have, bv);
+		if (have && conf > nconf) {
+			conf = nconf; depth = hd; normal = hn; bestViews = bv;
+			if (isRefine) {
+				pa = na; pb = nb;
+				++idxScale;
+				scaleRange = pow2neg(idxScale);
 			}
 		}
 	}
+	if (!live)
+		return;
 	const bool same = depth == pl.w && normal.x == pl.x && normal.y == pl.y && normal.z == pl.z;
 	P.plane[idx] = make_float4(normal.x, normal.y, normal.z, depth);
 	P.cost[idx] = (same && P.skipUnchanged) ? -conf : conf;
 	if (P.bestViews) P.bestViews[idx] = bestViews;
+}
+
+// MINB: resident CTAs per SM the register allocation aims at: 3 (80 registers, the default) or 4 (64 registers: one more CTA of
+// latency hiding against more spill traffic — b200mvs_debug.sweepFourCtas, measured in profiles/pm_4ctas_r02.txt: slower).
+// TMEM: SWEEP_TMEM_COLS columns per CTA, so 3 or 4 resident CTAs fit the 512 columns of an SM whichever launches they belong to.
+template <bool PACK, bool GEOM, int MINB>
+__global__ void __launch_bounds__(BLOCK_X*BLOCK_Y, MINB)
+pm_sweep_kernel(const __grid_constant__ PMParams P, const __grid_constant__ CUtensorMap tmapRef)
+{
+	extern __shared__ __align__(128) unsigned char smemRaw[];
+	// [ reference tile | mbarrier | TMEM address ]
+	float* tile = (float*)smemRaw;
+	uint64_t* bar = (uint64_t*)(tile + TILE_W*TILE_H);
+	uint32_t* sTmem = (uint32_t*)(bar+1);
+	const int tid = threadIdx.y*BLOCK_X + threadIdx.x, warp = tid>>5;
+	if (warp == 0) {
+		asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(sTmem)), "r"(SWEEP_TMEM_COLS) : "memory");
+		asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+	}
+	if (P.tma && tid == 32) {
+		mbar_init(bar, 1);
+		asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); // make the init visible to the async proxy
+	}
+	asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+	__syncthreads();
+	asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+	const uint32_t tmem = *sTmem + ((uint32_t)(32*(warp&3))<<16) + (warp >= 4 ? 64u : 0u);
+	if (P.tma) {
+		if (tid == 0) {
+			mbar_expect_tx(bar, TILE_BYTES);
+			tma_load_2d(tile, &tmapRef, (int)blockIdx.x*(2*BLOCK_X)-PM_HALF, (int)blockIdx.y*BLOCK_Y-PM_HALF, bar);
+		}
+		mbar_wait(bar, 0);
+	}
+	const int y = blockIdx.y*BLOCK_Y + threadIdx.y;
+	const int x = blockIdx.x*(2*BLOCK_X) + 2*threadIdx.x + ((y+P.colour)&1);
+	const bool live = x >= PM_HALF && y >= PM_HALF && x < P.W-PM_HALF && y < P.H-PM_HALF &&
+		!(P.mask && P.mask[(size_t)y*P.maskPitch + x] == 0);
+	if (__any_sync(0xFFFFFFFFu, live))   // warp-uniform: a warp without a pixel to update has nothing to do
+		sweep_pixel<PACK, GEOM>(P, tile, tmem, x, y, live);
+	asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+	__syncthreads();
+	if (warp == 0)
+		asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(*sTmem), "r"(SWEEP_TMEM_COLS) : "memory");
 }
 
 // pass C: threshold and convert cost to confidence (EndDepthMapTmp).  viewsMap: the (at most two) views of the
@@ -733,14 +803,10 @@ __global__ void pm_unpack_kernel(int n, const float4* __restrict__ plane, float*
 
 // ---- host launchers ---------------------------------------------------------------------
 constexpr size_t W_BYTES = (size_t)PM_TEXELS*NTHREADS*sizeof(float2);
-constexpr size_t SWEEP_SMEM = W_BYTES + TILE_BYTES + 16;
+constexpr size_t SWEEP_SMEM = TILE_BYTES + 16;   // tile, mbarrier, TMEM address: below the 48 KB default, no opt-in
 
 template <bool PACK, bool GEOM>
 cudaError_t configure_one() {
-	cudaError_t e = cudaFuncSetAttribute(pm_sweep_kernel<PACK, GEOM, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SWEEP_SMEM);
-	if (e != cudaSuccess) return e;
-	e = cudaFuncSetAttribute(pm_sweep_kernel<PACK, GEOM, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SWEEP_SMEM);
-	if (e != cudaSuccess) return e;
 	return cudaFuncSetAttribute(pm_score_kernel<PACK, GEOM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)W_BYTES);
 }
 
