@@ -250,6 +250,52 @@ int b200mvs_sgm_cross_check_device(b200mvs_ctx* ctx, int16_t* l2r, const int16_t
 int b200mvs_sgm_refine_device(b200mvs_ctx* ctx, const b200mvs_sgm_pixel* pixels, const uint16_t* accums,
 	int16_t* disparity, int nPixels, int subpixelSteps, void* stream);
 
+/* ---- coarse-to-fine (tSGM) matching of a rectified pair: the level loop of SemiGlobalMatcher::Match(scene, idxImage, numNeighbors,
+ * minResolution) (libs/MVS/SemiGlobalMatcher.cpp:584-718), the reference's default SGM path, between StereoRectifyImages and
+ * ExportDisparityDataRawFull.  Levels at 1/2^L .. 1/2, 1 of the full resolution: the coarsest level matches inside ranges derived
+ * from a seed disparity map, every finer level inside per-pixel ranges of at most 64 disparities derived from the level below, so
+ * the total disparity span is not limited to 256.
+ * b200mvs_sgm_tsgm_levels: number of levels (computeMaxResolution, libs/Common/Types.inl:2459-2477, minResolution > 0) and the size of
+ * the seed: computeResize(coarsest level, 0.5) minus 6 in each dimension (234 x 129 for 1920 x 1080). */
+int b200mvs_sgm_tsgm_levels(int width, int height, int minResolution, int* nLevels, int* seedWidth, int* seedHeight);
+
+/* DEVICE pointers, work on `stream` (NULL = the context's stream).  Images as b200mvs_sgm_match plus the right BGR image; masks
+ * (nullable = all valid): width x height bytes, 0 = invalid (StereoRectifyImages); maskWidth / maskHeight must equal width / height
+ * when a mask is given.  seed (nullable = all unknown): seedWidth x seedHeight int16 disparities at half the coarsest scale,
+ * 32767 = unknown.  nSpeckleSize: OPTDENSE::nSpeckleSize (100); subpixelSteps: 4; prm NULL = defaults.  Outputs over the
+ * (width-6) x (height-6) valid region: the refined left disparity x subpixelSteps (32767 = none) and the cost of the last left match.
+ * Synchronises the stream once per match (two per level), where the ragged cost volume is sized from the pixel map; when a match
+ * took the wave-front aggregation, once more to read its timeout flag.  stats != NULL: also at the end.  Scratch is grow-only on
+ * the context.  B200MVS_ERR_ARG for wrong seed or mask sizes, or an image too small for minResolution. */
+int b200mvs_sgm_match_tsgm_device(b200mvs_ctx* ctx, const float* leftGray, const uint8_t* leftBGR, const float* rightGray, const uint8_t* rightBGR,
+	int width, int height, const uint8_t* leftMask, const uint8_t* rightMask, int maskWidth, int maskHeight,
+	const int16_t* seed, int seedWidth, int seedHeight, int minResolution, int nSpeckleSize, int subpixelSteps,
+	const b200mvs_sgm_params* prm, int16_t* disparity, uint16_t* cost, void* stream, b200mvs_stats* stats);
+/* Same with HOST buffers: copies in, runs the device form on the context's stream, copies out. */
+int b200mvs_sgm_match_tsgm(b200mvs_ctx* ctx, const float* leftGray, const uint8_t* leftBGR, const float* rightGray, const uint8_t* rightBGR,
+	int width, int height, const uint8_t* leftMask, const uint8_t* rightMask, int maskWidth, int maskHeight,
+	const int16_t* seed, int seedWidth, int seedHeight, int minResolution, int nSpeckleSize, int subpixelSteps,
+	const b200mvs_sgm_params* prm, int16_t* disparity, uint16_t* cost, b200mvs_stats* stats);
+
+/* building blocks of the level loop (DEVICE pointers) */
+/* Disparity2RangeMap (SemiGlobalMatcher.cpp:1350-1444): ranges at twice the scale of `disparity` (width x height) over the finer
+ * valid region `mask` (maskWidth >= 2 width + 4, maskHeight >= 2 height + 2); pixels receives maskWidth x maskHeight records.
+ * Synchronises `stream` to return *numCosts and *maxNumDisp (nullable). */
+int b200mvs_sgm_range_map_device(b200mvs_ctx* ctx, const int16_t* disparity, int width, int height, const uint8_t* mask, int maskWidth, int maskHeight,
+	int minNumDisp, int minNumDispInvalid, b200mvs_sgm_pixel* pixels, uint64_t* numCosts, int* maxNumDisp, void* stream);
+/* FlipDirection (SemiGlobalMatcher.cpp:1630-1657): r2l = NO_DISP, every valid l2r(r,c) = d writes -d to r2l(r, c+d-1 .. c+d+1);
+ * where writes overlap the larger source column wins */
+int b200mvs_sgm_flip_direction_device(b200mvs_ctx* ctx, const int16_t* l2r, int16_t* r2l, int width, int height, void* stream);
+/* cv::filterSpeckles(disparity, newVal, maxSpeckleSize, maxDiff) on int16, in place */
+int b200mvs_sgm_filter_speckles_device(b200mvs_ctx* ctx, int16_t* disparity, int width, int height, int newVal, int maxSpeckleSize, int maxDiff, void* stream);
+/* ExtractMask (SemiGlobalMatcher.cpp:1518-1575): mask (same size) updated in place */
+int b200mvs_sgm_extract_mask_device(b200mvs_ctx* ctx, const int16_t* disparity, uint8_t* mask, int width, int height, int thValid, void* stream);
+/* UpscaleMask (SemiGlobalMatcher.cpp:1662-1690) into mask2x (width2 x height2) */
+int b200mvs_sgm_upscale_mask_device(b200mvs_ctx* ctx, const uint8_t* mask, int width, int height, uint8_t* mask2x, int width2, int height2, void* stream);
+/* cv::resize(image, Size(), 1./factor, 1./factor, INTER_AREA) of a 3-channel 8-bit image (integer factor >= 2); `resized` holds
+ * cvRound(width/factor) x cvRound(height/factor) pixels */
+int b200mvs_resize_area_bgr8_device(b200mvs_ctx* ctx, const uint8_t* image, int width, int height, int factor, uint8_t* resized, void* stream);
+
 /* ---- depth-map post-processing after the estimation (SURVEY.md §8(f) rank 2) -----------------
  * DepthMapsData::FilterDepthMap / RemoveSmallSegments / GapInterpolation
  * (libs/MVS/SceneDensify.cpp:1050-1299, 810-900, 904-1045).  Maps are contiguous row-major float

@@ -74,6 +74,17 @@ cudaError_t rs_launch_nearest(const float* src, int sw, int sh, int ch, float* d
 cudaError_t rs_launch_nearest_u8(const uint8_t* src, int sw, int sh, int spitch, uint8_t* dst, int dw, int dh, cudaStream_t s);
 cudaError_t rs_launch_to_gray(const uint8_t* src, int w, int h, int sstride, int channels, int bgr, float* dst, int dpitch, cudaStream_t s);
 cudaError_t rs_launch_plane_up(const float4* src, int sw, int sh, float4* dst, float* prior, int dw, int dh, bool nearestDepth, cudaStream_t s);
+// coarse-to-fine SGM steps (sgm_tsgm.cu)
+size_t ts_range_scratch_bytes(int mw, int mh);
+cudaError_t ts_launch_range_map(const int16_t* D, int dw, int dh, const uint8_t* M, int mw, int mh, int minNumDisp, int minNumDispInvalid,
+	uint32_t* range, void* scratch, void* pixels, unsigned long long* stat, cudaStream_t s);
+cudaError_t ts_launch_flip(const int16_t* l2r, int16_t* r2l, int w, int h, uint32_t* key, cudaStream_t s);
+cudaError_t ts_launch_filter_speckles(int16_t* img, int w, int h, int newVal, int maxSize, int maxDiff, int* labels, int* sizes, cudaStream_t s);
+int ts_filter_speckles_launches(int w, int h);
+cudaError_t ts_launch_extract_mask(const int16_t* disp, uint8_t* mask, int w, int h, int thValid, cudaStream_t s);
+cudaError_t ts_launch_upscale_mask(const uint8_t* m, int w, int h, uint8_t* m2, int w2, int h2, cudaStream_t s);
+cudaError_t ts_launch_resize_area_u8(const uint8_t* src, int sw, int sh, int ch, int f, uint8_t* dst, int dw, int dh, cudaStream_t s);
+cudaError_t ts_launch_fill_i16(int16_t* p, size_t n, int16_t v, cudaStream_t s);
 
 namespace {
 
@@ -151,6 +162,9 @@ struct b200mvs_ctx {
 	cudaStream_t sgSide[7] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // side streams of the ragged aggregation
 	cudaEvent_t sgJoin[7] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr}, sgFork = nullptr;
 	const void* sgLastPx = nullptr; uint64_t sgLastNum = 0; // pixel map / size of the volume in sgAccums (b200mvs_sgm_refine_device check)
+	bool sgFrontRan = false;                  // the last match aggregated with the wave-front kernel
+	// coarse-to-fine SGM (b200mvs_sgm_match_tsgm_device): pyramid level images, range-map scratch, pixel map, level maps
+	DevBuf tsLG, tsRG, tsLC, tsRC, tsRange, tsScratch, tsStat, tsPx, tsDisp, tsMask, tsLab, tsCost;
 	DevBuf fltZ, fltIn, fltOutD, fltOutC;     // FilterDepthMap: z-buffer keys, staged maps (host API), outputs
 	DevBuf ppA, ppB, ppD, ppN, ppC;           // RemoveSmallSegments labels/sizes, GapInterpolation temporaries, staging
 	DevBuf ppK, ppArcs, ppPatch;              // RemoveSmallSegments: seed keys, one-way edges (+ counter), patched segment sizes
@@ -595,6 +609,8 @@ int b200mvs_destroy(b200mvs_ctx* c) {
 	for (auto e: c->sweepEv) cudaEventDestroy(e);
 	c->sgL.release(); c->sgC.release(); c->sgR.release(); c->sgPx.release(); c->sgCosts.release(); c->sgAccums.release(); c->sgAccums2.release();
 	c->sgDisp.release(); c->sgCost.release(); c->sgMax.release();
+	for (DevBuf* b: {&c->tsLG, &c->tsRG, &c->tsLC, &c->tsRC, &c->tsRange, &c->tsScratch, &c->tsStat, &c->tsPx, &c->tsDisp, &c->tsMask, &c->tsLab, &c->tsCost})
+		b->release();
 	for (auto& fp: c->sgFront) { fp.items.release(); fp.need.release(); }
 	c->sgFrontCtl.release(); c->sgFrontState.release(); c->sgFrontMeta.release();
 	for (int i = 0; i < 7; ++i) { if (c->sgSide[i]) cudaStreamDestroy(c->sgSide[i]); if (c->sgJoin[i]) cudaEventDestroy(c->sgJoin[i]); }
@@ -911,9 +927,11 @@ int b200mvs_pm_finalize(b200mvs_ctx* ctx, int width, int height, float keep, con
 // ---- SGM --------------------------------------------------------------------------------------
 void b200mvs_sgm_default_params(b200mvs_sgm_params* p) { p->P1 = 3; p->P2 = 4; p->P2alpha = 14.f; p->P2beta = 38.f; }
 
-int b200mvs_sgm_match_device(b200mvs_ctx* ctx, const float* leftGray, const uint8_t* leftBGR, const float* rightGray,
+namespace {
+// b200mvs_sgm_match_device; known8 != NULL: the pixel-map statistics of sgm_launch_maxdisp, already read back by the caller
+int sgm_match(b200mvs_ctx* ctx, const float* leftGray, const uint8_t* leftBGR, const float* rightGray,
 	int width, int height, const b200mvs_sgm_pixel* pixels, uint64_t numCosts, const b200mvs_sgm_params* prm,
-	int stages, uint8_t* costs, uint16_t* accums, int16_t* disparity, uint16_t* cost, void* stream, b200mvs_stats* stats)
+	int stages, uint8_t* costs, uint16_t* accums, int16_t* disparity, uint16_t* cost, void* stream, b200mvs_stats* stats, const int* known8)
 {
 	if (!ctx) return B200MVS_ERR_ARG;
 	if (!leftGray || !leftBGR || !rightGray || !pixels || width <= 6 || height <= 6 || numCosts == 0)
@@ -948,10 +966,13 @@ int b200mvs_sgm_match_device(b200mvs_ctx* ctx, const float* leftGray, const uint
 	if (stats) CK(cudaEventRecord(ctx->ev0, s));
 	if (stages & 7) {
 		// the warp-per-scanline kernel keeps one line of at most sgm_max_disparities() values
-		CK(ctx->sgMax.reserve(8*sizeof(int)));
-		CK(sgm_launch_maxdisp(P.px, P.vw*P.vh, numCosts, ctx->sgMax.as<int>(), s)); ctx->launches += 2;
-		CK(cudaMemcpyAsync(st8, ctx->sgMax.p, 8*sizeof(int), cudaMemcpyDeviceToHost, s));
-		CK(cudaStreamSynchronize(s));
+		if (known8) memcpy(st8, known8, sizeof(st8));
+		else {
+			CK(ctx->sgMax.reserve(8*sizeof(int)));
+			CK(sgm_launch_maxdisp(P.px, P.vw*P.vh, numCosts, ctx->sgMax.as<int>(), s)); ctx->launches += 2;
+			CK(cudaMemcpyAsync(st8, ctx->sgMax.p, 8*sizeof(int), cudaMemcpyDeviceToHost, s));
+			CK(cudaStreamSynchronize(s));
+		}
 		if (st8[7])
 			return fail(ctx, B200MVS_ERR_ARG, "sgm: a pixel's slice [idx, idx+dmax-dmin) ends beyond numCosts");
 		if (st8[0] > sgm_max_disparities())
@@ -1016,7 +1037,7 @@ int b200mvs_sgm_match_device(b200mvs_ctx* ctx, const float* leftGray, const uint
 			++ctx->launches;
 		}
 	}
-	if (stages & 2) { ctx->sgLastPx = (accums == ctx->sgAccums.as<uint16_t>()) ? (const void*)pixels : nullptr; ctx->sgLastNum = numCosts; }
+	if (stages & 2) { ctx->sgLastPx = (accums == ctx->sgAccums.as<uint16_t>()) ? (const void*)pixels : nullptr; ctx->sgLastNum = numCosts; ctx->sgFrontRan = front; }
 	if (stages & 4) {
 		const bool denseWta = uniform && (st8[0] & 15) == 0 && !st8[6] && !((uintptr_t)P.accums & 15);
 		if (denseWta) CK(sgm_launch_wta_uniform(P, twoVolumes ? ctx->sgAccums2.as<uint16_t>() : nullptr, st8[1], st8[0], disparity, cost, s));
@@ -1039,6 +1060,15 @@ int b200mvs_sgm_match_device(b200mvs_ctx* ctx, const float* leftGray, const uint
 		}
 	}
 	return B200MVS_OK;
+}
+} // namespace
+
+int b200mvs_sgm_match_device(b200mvs_ctx* ctx, const float* leftGray, const uint8_t* leftBGR, const float* rightGray,
+	int width, int height, const b200mvs_sgm_pixel* pixels, uint64_t numCosts, const b200mvs_sgm_params* prm,
+	int stages, uint8_t* costs, uint16_t* accums, int16_t* disparity, uint16_t* cost, void* stream, b200mvs_stats* stats)
+{
+	return sgm_match(ctx, leftGray, leftBGR, rightGray, width, height, pixels, numCosts, prm, stages, costs, accums, disparity, cost,
+		stream, stats, nullptr);
 }
 
 int b200mvs_sgm_match(b200mvs_ctx* ctx, const float* leftGray, const uint8_t* leftBGR, const float* rightGray,
@@ -1093,6 +1123,318 @@ int b200mvs_sgm_refine_device(b200mvs_ctx* ctx, const b200mvs_sgm_pixel* pixels,
 	if (subpixelSteps <= 1) return B200MVS_OK;
 	CK(cudaSetDevice(ctx->device));
 	CK(sgm_launch_refine((const SGMPixel*)pixels, accums, disparity, nPixels, subpixelSteps, stream ? (cudaStream_t)stream : ctx->stream));
+	return B200MVS_OK;
+}
+
+// ---- coarse-to-fine (tSGM) matching of a rectified pair: the level loop of SemiGlobalMatcher::Match(scene, ...) ----
+// (libs/MVS/SemiGlobalMatcher.cpp:584-718; the per-level steps are in sgm_tsgm.cu, the matches are sgm_match)
+namespace {
+
+inline int cv_round(double v) { return (int)std::nearbyint(v); }   // cv::saturate_cast<int>(double)
+
+// computeMaxResolution (libs/Common/Types.inl:2459-2477) with level = 8, scale = 1/max(2, 2^level) (SemiGlobalMatcher.cpp:584-589);
+// the seed is the valid region of computeResize(coarsest level, 0.5) (:620-624)
+void tsgm_levels(int width, int height, int minResolution, int& nLevels, int& seedWidth, int& seedHeight) {
+	const unsigned imageSize = (unsigned)std::max(width, height);
+	unsigned level = 8;
+	if ((imageSize >> level) < (unsigned)minResolution) {
+		level = 0;
+		while ((imageSize >> (level+1)) >= (unsigned)minResolution)
+			++level;
+	}
+	const int L = (int)std::max(1u, level);
+	nLevels = L+1;
+	const int cw = cv_round(width/(double)(1 << L)), ch = cv_round(height/(double)(1 << L));
+	seedWidth = cv_round(cw*0.5)-6; seedHeight = cv_round(ch*0.5)-6;
+}
+
+// Disparity2RangeMap's layout needs the fine valid region to reach past 2 x the coarse map plus the 3-pixel offset
+inline bool range_sizes_ok(int dw, int dh, int mw, int mh) { return dw > 0 && dh > 0 && mw >= 2*dw+4 && mh >= 2*dh+2 && mw < 32768; }
+
+// Disparity2RangeMap into `pixels`; with st8 != NULL also the statistics the match needs (sgm_launch_maxdisp).  One read-back:
+// the volume of the following match is sized from it.
+int ts_range_map(b200mvs_ctx* ctx, const int16_t* D, int dw, int dh, const uint8_t* M, int mw, int mh, int minND, int minNDI,
+	void* pixels, uint64_t& numCosts, int& maxNumDisp, int* st8, cudaStream_t s)
+{
+	CK(ctx->tsRange.reserve((size_t)dw*dh*4));
+	CK(ctx->tsScratch.reserve(ts_range_scratch_bytes(mw, mh)));
+	CK(ctx->tsStat.reserve(64));
+	unsigned long long* stat = ctx->tsStat.as<unsigned long long>();
+	CK(ts_launch_range_map(D, dw, dh, M, mw, mh, minND, minNDI, ctx->tsRange.as<uint32_t>(), ctx->tsScratch.p, pixels, stat, s));
+	ctx->launches += 5;
+	if (st8) { CK(sgm_launch_maxdisp((const SGMPixel*)pixels, mw*mh, ~0ull, (int*)(stat+2), s)); ctx->launches += 2; }
+	unsigned long long host[6];
+	CK(cudaMemcpyAsync(host, stat, st8 ? 48 : 16, cudaMemcpyDeviceToHost, s));
+	CK(cudaStreamSynchronize(s));
+	numCosts = host[0];
+	maxNumDisp = (int)(uint32_t)host[1];
+	if (st8) memcpy(st8, host+2, 8*sizeof(int));
+	return B200MVS_OK;
+}
+
+// the wave-front aggregation flags a dependency wait that timed out (never in a correct schedule)
+int ts_check_front(b200mvs_ctx* ctx, cudaStream_t s) {
+	if (!ctx->sgFrontRan) return B200MVS_OK;
+	int err = 0;
+	CK(cudaMemcpyAsync(&err, ctx->sgFrontCtl.as<int>()+1, sizeof(int), cudaMemcpyDeviceToHost, s));
+	CK(cudaStreamSynchronize(s));
+	if (err) return fail(ctx, B200MVS_ERR_CUDA, "sgm: the wave-front aggregation timed out waiting for a predecessor");
+	return B200MVS_OK;
+}
+
+} // namespace
+
+int b200mvs_sgm_tsgm_levels(int width, int height, int minResolution, int* nLevels, int* seedWidth, int* seedHeight) {
+	if (!nLevels || !seedWidth || !seedHeight || width <= 0 || height <= 0 || minResolution <= 0) return B200MVS_ERR_ARG;
+	tsgm_levels(width, height, minResolution, *nLevels, *seedWidth, *seedHeight);
+	return B200MVS_OK;
+}
+
+int b200mvs_sgm_match_tsgm_device(b200mvs_ctx* ctx, const float* leftGray, const uint8_t* leftBGR, const float* rightGray, const uint8_t* rightBGR,
+	int width, int height, const uint8_t* leftMask, const uint8_t* rightMask, int maskWidth, int maskHeight,
+	const int16_t* seed, int seedWidth, int seedHeight, int minResolution, int nSpeckleSize, int subpixelSteps,
+	const b200mvs_sgm_params* prm, int16_t* disparity, uint16_t* cost, void* stream, b200mvs_stats* stats)
+{
+	if (!ctx) return B200MVS_ERR_ARG;
+	if (!leftGray || !leftBGR || !rightGray || !rightBGR || !disparity || !cost || width <= 6 || height <= 6 || width >= 32768 || height >= 32768)
+		return fail(ctx, B200MVS_ERR_ARG, "sgm tsgm: null image or output, or image size out of range");
+	if (minResolution <= 0 || nSpeckleSize < 0 || subpixelSteps < 1)
+		return fail(ctx, B200MVS_ERR_ARG, "sgm tsgm: needs minResolution > 0, nSpeckleSize >= 0, subpixelSteps >= 1");
+	if ((leftMask || rightMask) && (maskWidth != width || maskHeight != height))
+		return fail(ctx, B200MVS_ERR_ARG, "sgm tsgm: the masks must have the size of the images");
+	int nLevels, sw, sh;
+	tsgm_levels(width, height, minResolution, nLevels, sw, sh);
+	if (seed && (seedWidth != sw || seedHeight != sh))
+		return fail(ctx, B200MVS_ERR_ARG, "sgm tsgm: the seed must be computeResize(coarsest level, 0.5) minus 6 (b200mvs_sgm_tsgm_levels)");
+	{
+		int pw = sw, ph = sh;
+		for (int level = 0; level < nLevels; ++level) {
+			const int f = 1 << (nLevels-1-level);
+			const int vw = cv_round(width/(double)f)-6, vh = cv_round(height/(double)f)-6;
+			if (!range_sizes_ok(pw, ph, vw, vh))
+				return fail(ctx, B200MVS_ERR_ARG, "sgm tsgm: image too small for this minResolution");
+			pw = vw; ph = vh;
+		}
+	}
+	b200mvs_sgm_params def; b200mvs_sgm_default_params(&def);
+	if (!prm) prm = &def;
+	CK(cudaSetDevice(ctx->device));
+	cudaStream_t s = stream ? (cudaStream_t)stream : ctx->stream;
+	const auto t0 = std::chrono::steady_clock::now();
+	int launches = 0;
+	if (stats) CK(cudaEventRecord(ctx->ev0, s));
+	const size_t nv = (size_t)(width-6)*(height-6), n = (size_t)width*height;
+	// level images of every level below full resolution fit the half-resolution level
+	const size_t nHalf = (size_t)(cv_round(width*0.5)+1)*(cv_round(height*0.5)+1);
+	CK(ctx->tsLG.reserve(nHalf*4)); CK(ctx->tsRG.reserve(nHalf*4)); CK(ctx->tsLC.reserve(nHalf*3)); CK(ctx->tsRC.reserve(nHalf*3));
+	CK(ctx->tsDisp.reserve(4*nv*2)); CK(ctx->tsMask.reserve(4*nv+n)); CK(ctx->tsLab.reserve(2*nv*4));
+	CK(ctx->tsCost.reserve(nv*2)); CK(ctx->tsPx.reserve(nv*sizeof(SGMPixel)));
+	int16_t* dbuf[2] = {ctx->tsDisp.as<int16_t>(), ctx->tsDisp.as<int16_t>()+nv};
+	int16_t* rFlip = ctx->tsDisp.as<int16_t>()+2*nv;
+	int16_t* rD = ctx->tsDisp.as<int16_t>()+3*nv;
+	uint8_t* mbuf[2][2] = {{ctx->tsMask.as<uint8_t>(), ctx->tsMask.as<uint8_t>()+nv}, {ctx->tsMask.as<uint8_t>()+2*nv, ctx->tsMask.as<uint8_t>()+3*nv}};
+	uint8_t* maskTmp = ctx->tsMask.as<uint8_t>()+4*nv;
+	int* lab = ctx->tsLab.as<int>();
+	void* px = ctx->tsPx.p;
+	const int16_t* lPrev = seed;
+	if (!seed) { CK(ts_launch_fill_i16(dbuf[0], (size_t)sw*sh, 32767, s)); ++launches; lPrev = dbuf[0]; }
+	int pw = sw, ph = sh, cur = 0;   // size of the previous level's maps, mask ping-pong slot
+	for (int level = 0; level < nLevels; ++level) {
+		const int f = 1 << (nLevels-1-level);
+		const bool first = level == 0, last = level+1 == nLevels;
+		// ViewData::GetImage(scale) (SemiGlobalMatcher.h:127-142)
+		int lw = width, lh = height;
+		const float *LG = leftGray, *RG = rightGray; const uint8_t *LC = leftBGR, *RC = rightBGR;
+		if (f > 1) {
+			lw = cv_round(width/(double)f); lh = cv_round(height/(double)f);
+			CK(rs_launch_area(leftGray, width, height, width, ctx->tsLG.as<float>(), lw, lh, f, f, s));
+			CK(rs_launch_area(rightGray, width, height, width, ctx->tsRG.as<float>(), lw, lh, f, f, s));
+			CK(ts_launch_resize_area_u8(leftBGR, width, height, 3, f, ctx->tsLC.as<uint8_t>(), lw, lh, s));
+			CK(ts_launch_resize_area_u8(rightBGR, width, height, 3, f, ctx->tsRC.as<uint8_t>(), lw, lh, s));
+			launches += 4;
+			LG = ctx->tsLG.as<float>(); RG = ctx->tsRG.as<float>(); LC = ctx->tsLC.as<uint8_t>(); RC = ctx->tsRC.as<uint8_t>();
+		}
+		const int vw = lw-6, vh = lh-6;
+		const size_t nl = (size_t)vw*vh;
+		uint8_t* lM = mbuf[cur^1][0];
+		uint8_t* rM = mbuf[cur^1][1];
+		for (int m = 0; m < 2; ++m) {
+			uint8_t* dst = m == 0 ? lM : rM;
+			const uint8_t* src = m == 0 ? leftMask : rightMask;
+			if (!first) { CK(ts_launch_upscale_mask(mbuf[cur][m], pw, ph, dst, vw, vh, s)); ++launches; }
+			else if (!src) CK(cudaMemsetAsync(dst, 255, nl, s));
+			else {
+				// NEAREST to the level size, then the valid ROI (:626-631)
+				CK(rs_launch_nearest_u8(src, width, height, width, maskTmp, lw, lh, s)); ++launches;
+				CK(cudaMemcpy2DAsync(dst, vw, maskTmp+3*lw+3, lw, vw, vh, cudaMemcpyDeviceToDevice, s));
+			}
+		}
+		cur ^= 1;
+		const int minND = first ? 11 : 5, minNDI = first ? 33 : 7;
+		int16_t* lCur = last ? disparity : (lPrev == dbuf[0] ? dbuf[1] : dbuf[0]);
+		uint16_t* lCost = last ? cost : ctx->tsCost.as<uint16_t>();
+		int st8[8]; uint64_t numCosts; int maxND; int rc;
+		auto match = [&](const float* a, const uint8_t* ac, const float* b, int16_t* d, uint16_t* c) -> int {
+			if (numCosts == 0) {
+				// every pixel masked out: the winner-takes-all of the reference leaves NO_DISP / NO_ACCUMCOST
+				CK(ts_launch_fill_i16(d, nl, 32767, s)); ++launches;
+				CK(cudaMemsetAsync(c, 0xFF, nl*2, s));
+				return B200MVS_OK;
+			}
+			const int r = sgm_match(ctx, a, ac, b, lw, lh, (const b200mvs_sgm_pixel*)px, numCosts, prm, 7, nullptr, nullptr, d, c, s, nullptr, st8);
+			launches += ctx->launches;
+			return r ? r : ts_check_front(ctx, s);
+		};
+		// right -> left: FlipDirection, Disparity2RangeMap, Match(right, left) (:641-642, 672)
+		CK(ts_launch_flip(lPrev, rFlip, pw, ph, (uint32_t*)lab, s)); launches += 2;
+		ctx->launches = 0;
+		if ((rc = ts_range_map(ctx, rFlip, pw, ph, rM, vw, vh, minND, minNDI, px, numCosts, maxND, st8, s))) return rc;
+		launches += ctx->launches;
+		if ((rc = match(RG, RC, LG, rD, ctx->tsCost.as<uint16_t>()))) return rc;
+		// left -> right (:675-685)
+		ctx->launches = 0;
+		if ((rc = ts_range_map(ctx, lPrev, pw, ph, lM, vw, vh, minND, minNDI, px, numCosts, maxND, st8, s))) return rc;
+		launches += ctx->launches;
+		if ((rc = match(LG, LC, RG, lCur, lCost))) return rc;
+		if (first) {
+			// :698-706; the second cross-check reads the already-checked left map
+			CK(sgm_launch_cross_check(lCur, rD, vw, vh, 1, s));
+			CK(sgm_launch_cross_check(rD, lCur, vw, vh, 1, s));
+			CK(ts_launch_filter_speckles(lCur, vw, vh, 32767, nSpeckleSize, 5, lab, lab+nv, s));
+			CK(ts_launch_filter_speckles(rD, vw, vh, 32767, nSpeckleSize, 5, lab, lab+nv, s));
+			CK(ts_launch_extract_mask(lCur, lM, vw, vh, 3, s));
+			CK(ts_launch_extract_mask(rD, rM, vw, vh, 3, s));
+			launches += 4 + 2*ts_filter_speckles_launches(vw, vh);
+		} else {
+			CK(sgm_launch_cross_check(lCur, rD, vw, vh, 1, s)); ++launches;
+		}
+		lPrev = lCur; pw = vw; ph = vh;
+		if (last && numCosts > 0 && subpixelSteps > 1) {
+			// RefineDisparityMap with the pixel map and the accumulated costs of this last left match (:718)
+			CK(sgm_launch_refine((const SGMPixel*)px, ctx->sgAccums.as<uint16_t>(), disparity, (int)nl, subpixelSteps, s)); ++launches;
+		}
+	}
+	ctx->sgLastPx = nullptr;
+	ctx->launches = launches;
+	if (stats) {
+		CK(cudaEventRecord(ctx->ev1, s));
+		CK(cudaStreamSynchronize(s));
+		float ms = 0; CK(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+		memset(stats, 0, sizeof(*stats));
+		stats->ms_device = ms;
+		stats->ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now()-t0).count();
+		stats->kernel_launches = launches; stats->levels = nLevels;
+	}
+	return B200MVS_OK;
+}
+
+int b200mvs_sgm_match_tsgm(b200mvs_ctx* ctx, const float* leftGray, const uint8_t* leftBGR, const float* rightGray, const uint8_t* rightBGR,
+	int width, int height, const uint8_t* leftMask, const uint8_t* rightMask, int maskWidth, int maskHeight,
+	const int16_t* seed, int seedWidth, int seedHeight, int minResolution, int nSpeckleSize, int subpixelSteps,
+	const b200mvs_sgm_params* prm, int16_t* disparity, uint16_t* cost, b200mvs_stats* stats)
+{
+	if (!ctx) return B200MVS_ERR_ARG;
+	if (!leftGray || !leftBGR || !rightGray || !rightBGR || !disparity || !cost || width <= 6 || height <= 6 || width >= 32768 || height >= 32768)
+		return fail(ctx, B200MVS_ERR_ARG, "sgm tsgm: null image or output, or image size out of range");
+	if ((leftMask || rightMask) && (maskWidth != width || maskHeight != height))
+		return fail(ctx, B200MVS_ERR_ARG, "sgm tsgm: the masks must have the size of the images");
+	int nLevels, sw, sh;
+	if (minResolution <= 0) return fail(ctx, B200MVS_ERR_ARG, "sgm tsgm: needs minResolution > 0");
+	tsgm_levels(width, height, minResolution, nLevels, sw, sh);
+	if (seed && (seedWidth != sw || seedHeight != sh))
+		return fail(ctx, B200MVS_ERR_ARG, "sgm tsgm: the seed must be computeResize(coarsest level, 0.5) minus 6 (b200mvs_sgm_tsgm_levels)");
+	CK(cudaSetDevice(ctx->device));
+	cudaStream_t s = ctx->stream;
+	const auto t0 = std::chrono::steady_clock::now();
+	const size_t n = (size_t)width*height, nv = (size_t)(width-6)*(height-6), ns = seed ? (size_t)sw*sh : 0;
+	CK(ctx->sgL.reserve(n*4)); CK(ctx->sgR.reserve(n*4)); CK(ctx->sgC.reserve(n*6+2*n+ns*2));
+	CK(ctx->sgDisp.reserve(nv*2)); CK(ctx->sgCost.reserve(nv*2));
+	uint8_t* lc = ctx->sgC.as<uint8_t>(); uint8_t* rc = lc+3*n; uint8_t* lm = rc+3*n; uint8_t* rm = lm+n;
+	int16_t* sd = (int16_t*)(rm+n);
+	CK(cudaMemcpyAsync(ctx->sgL.p, leftGray, n*4, cudaMemcpyHostToDevice, s));
+	CK(cudaMemcpyAsync(ctx->sgR.p, rightGray, n*4, cudaMemcpyHostToDevice, s));
+	CK(cudaMemcpyAsync(lc, leftBGR, n*3, cudaMemcpyHostToDevice, s));
+	CK(cudaMemcpyAsync(rc, rightBGR, n*3, cudaMemcpyHostToDevice, s));
+	if (leftMask) CK(cudaMemcpyAsync(lm, leftMask, n, cudaMemcpyHostToDevice, s));
+	if (rightMask) CK(cudaMemcpyAsync(rm, rightMask, n, cudaMemcpyHostToDevice, s));
+	if (seed) CK(cudaMemcpyAsync(sd, seed, ns*2, cudaMemcpyHostToDevice, s));
+	b200mvs_stats st;
+	int r = b200mvs_sgm_match_tsgm_device(ctx, ctx->sgL.as<float>(), lc, ctx->sgR.as<float>(), rc, width, height,
+		leftMask ? lm : nullptr, rightMask ? rm : nullptr, maskWidth, maskHeight, seed ? sd : nullptr, seedWidth, seedHeight,
+		minResolution, nSpeckleSize, subpixelSteps, prm, ctx->sgDisp.as<int16_t>(), ctx->sgCost.as<uint16_t>(), s, &st);
+	if (r) return r;
+	CK(cudaMemcpyAsync(disparity, ctx->sgDisp.p, nv*2, cudaMemcpyDeviceToHost, s));
+	CK(cudaMemcpyAsync(cost, ctx->sgCost.p, nv*2, cudaMemcpyDeviceToHost, s));
+	CK(cudaStreamSynchronize(s));
+	if (stats) {
+		*stats = st;
+		stats->bytes_h2d = n*14 + (leftMask ? n : 0) + (rightMask ? n : 0) + ns*2; stats->bytes_d2h = nv*4;
+		stats->ms_total = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now()-t0).count();
+	}
+	return B200MVS_OK;
+}
+
+int b200mvs_sgm_range_map_device(b200mvs_ctx* ctx, const int16_t* disparity, int width, int height, const uint8_t* mask, int maskWidth, int maskHeight,
+	int minNumDisp, int minNumDispInvalid, b200mvs_sgm_pixel* pixels, uint64_t* numCosts, int* maxNumDisp, void* stream)
+{
+	if (!ctx) return B200MVS_ERR_ARG;
+	if (!disparity || !mask || !pixels || !range_sizes_ok(width, height, maskWidth, maskHeight))
+		return fail(ctx, B200MVS_ERR_ARG, "sgm range map: null pointer, or the mask is not at least (2w+4) x (2h+2)");
+	CK(cudaSetDevice(ctx->device));
+	uint64_t nc; int mx;
+	ctx->launches = 0;
+	const int rc = ts_range_map(ctx, disparity, width, height, mask, maskWidth, maskHeight, minNumDisp, minNumDispInvalid, pixels, nc, mx,
+		nullptr, stream ? (cudaStream_t)stream : ctx->stream);
+	if (rc) return rc;
+	if (numCosts) *numCosts = nc;
+	if (maxNumDisp) *maxNumDisp = mx;
+	return B200MVS_OK;
+}
+
+int b200mvs_sgm_flip_direction_device(b200mvs_ctx* ctx, const int16_t* l2r, int16_t* r2l, int width, int height, void* stream) {
+	if (!ctx) return B200MVS_ERR_ARG;
+	if (!l2r || !r2l || width <= 0 || height <= 0 || width >= 32768) return fail(ctx, B200MVS_ERR_ARG, "sgm flip: null pointer or size out of range");
+	CK(cudaSetDevice(ctx->device));
+	CK(ctx->tsLab.reserve((size_t)width*height*4));
+	CK(ts_launch_flip(l2r, r2l, width, height, ctx->tsLab.as<uint32_t>(), stream ? (cudaStream_t)stream : ctx->stream));
+	return B200MVS_OK;
+}
+
+int b200mvs_sgm_filter_speckles_device(b200mvs_ctx* ctx, int16_t* disparity, int width, int height, int newVal, int maxSpeckleSize, int maxDiff, void* stream) {
+	if (!ctx) return B200MVS_ERR_ARG;
+	if (!disparity || width <= 0 || height <= 0 || (size_t)width*height >= (1u << 31) || maxDiff < 0)
+		return fail(ctx, B200MVS_ERR_ARG, "sgm filter speckles: null map, size out of range or maxDiff < 0");
+	CK(cudaSetDevice(ctx->device));
+	const size_t n = (size_t)width*height;
+	CK(ctx->tsLab.reserve(n*8));
+	CK(ts_launch_filter_speckles(disparity, width, height, newVal, maxSpeckleSize, maxDiff, ctx->tsLab.as<int>(), ctx->tsLab.as<int>()+n,
+		stream ? (cudaStream_t)stream : ctx->stream));
+	return B200MVS_OK;
+}
+
+int b200mvs_sgm_extract_mask_device(b200mvs_ctx* ctx, const int16_t* disparity, uint8_t* mask, int width, int height, int thValid, void* stream) {
+	if (!ctx) return B200MVS_ERR_ARG;
+	if (!disparity || !mask || width <= 0 || height <= 0) return fail(ctx, B200MVS_ERR_ARG, "sgm extract mask: null pointer or empty map");
+	CK(cudaSetDevice(ctx->device));
+	CK(ts_launch_extract_mask(disparity, mask, width, height, thValid, stream ? (cudaStream_t)stream : ctx->stream));
+	return B200MVS_OK;
+}
+
+int b200mvs_sgm_upscale_mask_device(b200mvs_ctx* ctx, const uint8_t* mask, int width, int height, uint8_t* mask2x, int width2, int height2, void* stream) {
+	if (!ctx) return B200MVS_ERR_ARG;
+	if (!mask || !mask2x || width <= 0 || height <= 0 || width2 <= 0 || height2 <= 0) return fail(ctx, B200MVS_ERR_ARG, "sgm upscale mask: null pointer or empty map");
+	CK(cudaSetDevice(ctx->device));
+	CK(ts_launch_upscale_mask(mask, width, height, mask2x, width2, height2, stream ? (cudaStream_t)stream : ctx->stream));
+	return B200MVS_OK;
+}
+
+int b200mvs_resize_area_bgr8_device(b200mvs_ctx* ctx, const uint8_t* image, int width, int height, int factor, uint8_t* resized, void* stream) {
+	if (!ctx) return B200MVS_ERR_ARG;
+	if (!image || !resized || width <= 0 || height <= 0 || factor < 2) return fail(ctx, B200MVS_ERR_ARG, "resize area bgr8: null pointer, empty image or factor < 2");
+	const int dw = cv_round(width/(double)factor), dh = cv_round(height/(double)factor);
+	if (dw <= 0 || dh <= 0) return fail(ctx, B200MVS_ERR_ARG, "resize area bgr8: resized image is empty");
+	CK(cudaSetDevice(ctx->device));
+	CK(ts_launch_resize_area_u8(image, width, height, 3, factor, resized, dw, dh, stream ? (cudaStream_t)stream : ctx->stream));
 	return B200MVS_OK;
 }
 

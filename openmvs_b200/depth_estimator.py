@@ -141,6 +141,14 @@ def _is_torch(a) -> bool:
 	return type(a).__module__.startswith("torch")
 
 
+def _mask_size(leftMask, rightMask):
+	"""(height, width) shared by the given masks of a pair, (0, 0) without masks"""
+	shapes = {tuple(m.shape) for m in (leftMask, rightMask) if m is not None}
+	if len(shapes) > 1:
+		raise ValueError("left and right masks must have one size")
+	return shapes.pop() if shapes else (0, 0)
+
+
 def _make_views(images: List[ViewData]):
 	"""-> (ctypes View array, keepalive list, on_device flag)"""
 	n = len(images)
@@ -652,6 +660,115 @@ class SemiGlobalMatcher:
 		self.RefineDisparityMap(ldisp, pxl, None, subpixelSteps)  # accumulated costs of the last (left) match
 		torch.cuda.current_stream(dev).synchronize()
 		return ldisp, rdisp
+
+	# ---- coarse-to-fine (tSGM) matching, the reference's default SGM path ----
+	@staticmethod
+	def TsgmLevels(width: int, height: int, minResolution: int = 320):
+		"""-> (number of levels, seed width, seed height) of the coarse-to-fine loop (b200mvs_sgm_tsgm_levels)."""
+		lib = _lib.load()
+		o = [C.c_int() for _ in range(3)]
+		rc = lib.b200mvs_sgm_tsgm_levels(int(width), int(height), int(minResolution), *[C.byref(v) for v in o])
+		if rc != 0:
+			raise _lib.B200MVSError("b200mvs_sgm_tsgm_levels(%d, %d, %d) failed with status %d" % (width, height, minResolution, rc))
+		return tuple(v.value for v in o)
+
+	def MatchPyramidDevice(self, leftGray, leftColor, rightGray, rightColor, leftMask=None, rightMask=None, seed=None,
+			minResolution: int = 320, nSpeckleSize: int = 100, subpixelSteps: int = 4, sync: bool = True):
+		"""The level loop of SemiGlobalMatcher::Match(scene, ...) (libs/MVS/SemiGlobalMatcher.cpp:584-718) for one rectified pair on
+		CUDA tensors: gray float32 (H, W), colour uint8 (H, W, 3) BGR, masks uint8 (H, W) 0 = invalid (None = all valid), seed int16
+		of the size TsgmLevels gives (32767 = unknown; None = all unknown).  Returns (leftDisparity * subpixelSteps, cost) over the
+		(H-6, W-6) valid region as int16 tensors (NO_DISP = 32767; cost holds the uint16 bit pattern)."""
+		import torch
+		h, w = leftGray.shape
+		dev = leftGray.device
+		disp = torch.empty((h-6, w-6), dtype=torch.int16, device=dev)
+		cost = torch.empty((h-6, w-6), dtype=torch.int16, device=dev)
+		mh, mw = _mask_size(leftMask, rightMask)
+		sh, sw = seed.shape if seed is not None else (0, 0)
+		ptr = lambda t: t.data_ptr() if t is not None else None
+		rc = self._lib.b200mvs_sgm_match_tsgm_device(self._ctx, leftGray.data_ptr(), leftColor.data_ptr(), rightGray.data_ptr(),
+			rightColor.data_ptr(), w, h, ptr(leftMask), ptr(rightMask), mw, mh, ptr(seed), sw, sh, int(minResolution),
+			int(nSpeckleSize), int(subpixelSteps), C.byref(self.prm), disp.data_ptr(), cost.data_ptr(),
+			C.c_void_p(_stream_handle(dev)), C.byref(self.stats) if sync else None)
+		_lib.check(self._lib, self._ctx, rc, "b200mvs_sgm_match_tsgm_device")
+		return disp, cost
+
+	def MatchPyramid(self, leftGray, leftColor, rightGray, rightColor, leftMask=None, rightMask=None, seed=None,
+			minResolution: int = 320, nSpeckleSize: int = 100, subpixelSteps: int = 4):
+		"""Host form of MatchPyramidDevice on numpy arrays -> (leftDisparity * subpixelSteps int16, cost uint16)."""
+		lg = np.ascontiguousarray(leftGray, np.float32); rg = np.ascontiguousarray(rightGray, np.float32)
+		lc = np.ascontiguousarray(leftColor, np.uint8); rcol = np.ascontiguousarray(rightColor, np.uint8)
+		h, w = lg.shape
+		lm = None if leftMask is None else np.ascontiguousarray(leftMask, np.uint8)
+		rm = None if rightMask is None else np.ascontiguousarray(rightMask, np.uint8)
+		sd = None if seed is None else np.ascontiguousarray(seed, np.int16)
+		mh, mw = _mask_size(lm, rm)
+		sh, sw = sd.shape if sd is not None else (0, 0)
+		disp = np.zeros((h-6, w-6), np.int16); cost = np.zeros((h-6, w-6), np.uint16)
+		ptr = lambda a: a.ctypes.data if a is not None else None
+		rc = self._lib.b200mvs_sgm_match_tsgm(self._ctx, lg.ctypes.data, lc.ctypes.data, rg.ctypes.data, rcol.ctypes.data, w, h,
+			ptr(lm), ptr(rm), mw, mh, ptr(sd), sw, sh, int(minResolution), int(nSpeckleSize), int(subpixelSteps), C.byref(self.prm),
+			disp.ctypes.data, cost.ctypes.data, C.byref(self.stats))
+		_lib.check(self._lib, self._ctx, rc, "b200mvs_sgm_match_tsgm")
+		return disp, cost
+
+	def Disparity2RangeMap(self, disparityMap, maskMap, minNumDisp: int, minNumDispInvalid: int):
+		"""SemiGlobalMatcher::Disparity2RangeMap on CUDA tensors (int16 coarse map, uint8 fine mask) ->
+		(PixelMap as (n, 16) uint8 records, numCosts, maxNumDisp).  Synchronises the stream."""
+		import torch
+		h, w = disparityMap.shape
+		mh, mw = maskMap.shape
+		px = torch.empty((mh*mw, 16), dtype=torch.uint8, device=disparityMap.device)
+		nc = C.c_uint64(); mx = C.c_int()
+		rc = self._lib.b200mvs_sgm_range_map_device(self._ctx, disparityMap.data_ptr(), w, h, maskMap.data_ptr(), mw, mh, int(minNumDisp),
+			int(minNumDispInvalid), px.data_ptr(), C.byref(nc), C.byref(mx), C.c_void_p(_stream_handle(disparityMap.device)))
+		_lib.check(self._lib, self._ctx, rc, "b200mvs_sgm_range_map_device")
+		return px, int(nc.value), int(mx.value)
+
+	def FlipDirection(self, l2r):
+		"""SemiGlobalMatcher::FlipDirection: int16 CUDA tensor -> the right-to-left map."""
+		import torch
+		h, w = l2r.shape
+		r2l = torch.empty_like(l2r)
+		rc = self._lib.b200mvs_sgm_flip_direction_device(self._ctx, l2r.data_ptr(), r2l.data_ptr(), w, h, C.c_void_p(_stream_handle(l2r.device)))
+		_lib.check(self._lib, self._ctx, rc, "b200mvs_sgm_flip_direction_device")
+		return r2l
+
+	def FilterSpeckles(self, disparityMap, newVal: int = NO_DISP, maxSpeckleSize: int = 100, maxDiff: int = 5):
+		"""cv::filterSpeckles on an int16 CUDA tensor, in place."""
+		h, w = disparityMap.shape
+		rc = self._lib.b200mvs_sgm_filter_speckles_device(self._ctx, disparityMap.data_ptr(), w, h, int(newVal), int(maxSpeckleSize), int(maxDiff),
+			C.c_void_p(_stream_handle(disparityMap.device)))
+		_lib.check(self._lib, self._ctx, rc, "b200mvs_sgm_filter_speckles_device")
+		return disparityMap
+
+	def ExtractMask(self, disparityMap, maskMap, thValid: int = 3):
+		"""SemiGlobalMatcher::ExtractMask on CUDA tensors; maskMap (uint8) in place."""
+		h, w = disparityMap.shape
+		rc = self._lib.b200mvs_sgm_extract_mask_device(self._ctx, disparityMap.data_ptr(), maskMap.data_ptr(), w, h, int(thValid),
+			C.c_void_p(_stream_handle(disparityMap.device)))
+		_lib.check(self._lib, self._ctx, rc, "b200mvs_sgm_extract_mask_device")
+		return maskMap
+
+	def UpscaleMask(self, maskMap, width2: int, height2: int):
+		"""SemiGlobalMatcher::UpscaleMask: uint8 CUDA tensor -> mask of (height2, width2)."""
+		import torch
+		h, w = maskMap.shape
+		out = torch.empty((height2, width2), dtype=torch.uint8, device=maskMap.device)
+		rc = self._lib.b200mvs_sgm_upscale_mask_device(self._ctx, maskMap.data_ptr(), w, h, out.data_ptr(), int(width2), int(height2),
+			C.c_void_p(_stream_handle(maskMap.device)))
+		_lib.check(self._lib, self._ctx, rc, "b200mvs_sgm_upscale_mask_device")
+		return out
+
+	def ResizeAreaBGR8(self, image, factor: int):
+		"""cv::resize(image, Size(), 1/factor, 1/factor, INTER_AREA) of a uint8 (H, W, 3) CUDA tensor, integer factor."""
+		import torch
+		h, w = image.shape[:2]
+		out = torch.empty((int(round(h/factor)), int(round(w/factor)), 3), dtype=torch.uint8, device=image.device)
+		rc = self._lib.b200mvs_resize_area_bgr8_device(self._ctx, image.data_ptr(), w, h, int(factor), out.data_ptr(),
+			C.c_void_p(_stream_handle(image.device)))
+		_lib.check(self._lib, self._ctx, rc, "b200mvs_resize_area_bgr8_device")
+		return out
 
 
 @dataclasses.dataclass

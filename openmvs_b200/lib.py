@@ -96,6 +96,9 @@ SYMBOLS = [
 	"b200mvs_pm_pack", "b200mvs_pm_unpack", "b200mvs_pm_score", "b200mvs_pm_sweep", "b200mvs_pm_finalize",
 	"b200mvs_sgm_default_params", "b200mvs_sgm_match", "b200mvs_sgm_match_device",
 	"b200mvs_sgm_cross_check_device", "b200mvs_sgm_refine_device",
+	"b200mvs_sgm_tsgm_levels", "b200mvs_sgm_match_tsgm_device", "b200mvs_sgm_match_tsgm", "b200mvs_sgm_range_map_device",
+	"b200mvs_sgm_flip_direction_device", "b200mvs_sgm_filter_speckles_device", "b200mvs_sgm_extract_mask_device",
+	"b200mvs_sgm_upscale_mask_device", "b200mvs_resize_area_bgr8_device",
 	"b200mvs_filter_default_params", "b200mvs_filter_depth_map", "b200mvs_filter_depth_map_device",
 	"b200mvs_remove_small_segments", "b200mvs_remove_small_segments_device",
 	"b200mvs_gap_interpolation", "b200mvs_gap_interpolation_device",
@@ -163,6 +166,16 @@ def load(build_if_missing: bool = True):
 	lib.b200mvs_pointcloud_free.restype = None
 	lib.b200mvs_sgm_cross_check_device.argtypes = [P, P, P, C.c_int, C.c_int, C.c_int, P]
 	lib.b200mvs_sgm_refine_device.argtypes = [P, P, P, P, C.c_int, C.c_int, P]
+	I = C.c_int
+	lib.b200mvs_sgm_tsgm_levels.argtypes = [I, I, I, C.POINTER(I), C.POINTER(I), C.POINTER(I)]
+	lib.b200mvs_sgm_match_tsgm_device.argtypes = [P, P, P, P, P, I, I, P, P, I, I, P, I, I, I, I, I, C.POINTER(SgmParams), P, P, P, C.POINTER(Stats)]
+	lib.b200mvs_sgm_match_tsgm.argtypes = [P, P, P, P, P, I, I, P, P, I, I, P, I, I, I, I, I, C.POINTER(SgmParams), P, P, C.POINTER(Stats)]
+	lib.b200mvs_sgm_range_map_device.argtypes = [P, P, I, I, P, I, I, I, I, P, C.POINTER(C.c_uint64), C.POINTER(I), P]
+	lib.b200mvs_sgm_flip_direction_device.argtypes = [P, P, P, I, I, P]
+	lib.b200mvs_sgm_filter_speckles_device.argtypes = [P, P, I, I, I, I, I, P]
+	lib.b200mvs_sgm_extract_mask_device.argtypes = [P, P, P, I, I, I, P]
+	lib.b200mvs_sgm_upscale_mask_device.argtypes = [P, P, I, I, P, I, I, P]
+	lib.b200mvs_resize_area_bgr8_device.argtypes = [P, P, I, I, I, P, P]
 	lib.b200mvs_filter_default_params.argtypes = [C.POINTER(FilterParams)]
 	lib.b200mvs_filter_depth_map.argtypes = [P, C.POINTER(DMap), C.POINTER(DMap), C.c_int, C.POINTER(FilterParams), F, F, P, P,
 		C.POINTER(C.c_int), C.POINTER(Stats)]
